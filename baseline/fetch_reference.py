@@ -6,9 +6,7 @@ The reference (NVlabs/neuralrgbd) is pure Python with no setup.py / pyproject.to
 `pip install --target`: the "install" is a verbatim copy of its source tree (0.6 MB). baseline/_ref/ is git-ignored
 (never part of this repo's history) but NOT gpurun-ignored, so it travels to the GPU box, where /root/reference
 does not exist. It is used only by
-  * bench.py --impl reference / --impl reference-gpu   (the reference's own KVNET.forward, timed beside the engine),
-  * tests/test_gpu_dropin.py                           (the reference's own test_utils/test_KVNet.py:test driven
-                                                        through neuralrgbd_b200.install_as_reference_modules()).
+  * bench.py --impl reference / --impl reference-gpu   (the reference's own KVNET.forward, timed beside the engine).
 A MANIFEST with the sha256 of every copied file is written next to it so a reader can check nothing was edited.
 """
 import hashlib

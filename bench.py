@@ -2,6 +2,7 @@
 """bench.py - depth frames/s of the plane-sweep DPV hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config c1..c5] [--impl engine|reference|reference-gpu]
+                    [--dump-outputs DIR]
 
 Workloads = BASELINE.json configs (SURVEY 8d). `--config` picks one; the default c2 is the configuration the metric is
 quoted on (the driver's BENCH / SCALE runs use it), the others write the same JSON line for their shape:
@@ -33,6 +34,11 @@ cpu_baseline / --impl reference: the UNMODIFIED reference (baseline/_ref, copied
 
 N > 1 (torchrun): one process per GPU; frames (c1, c2, c5) / trajectory chunks (c3, c4) shard across ranks, weights are
 broadcast once over NCCL, no per-frame collective; value = all ranks' frames / max-over-ranks time.
+
+--dump-outputs DIR (engine arm, rank 0): what the last timed step returned, as DIR/<name>.npy in float32 - c1 the cost
+         volume; c2/c5 dmap_cur_refined, bv_cur, depth_lowres; c3/c4 the maps of the last streamed frame and the prior it
+         propagated (bv_predict_next). Inputs and weights are seeded, so the same arguments give the same inputs on every
+         run and two builds can be compared output for output.
 """
 import argparse
 import contextlib
@@ -123,6 +129,31 @@ def conv_traffic_per_launch():
         return float(json.load(open(os.path.join(ROOT, 'profiles', 'r2_conv_dram_traffic.json')))['traffic_bytes_per_launch'])
     except Exception:
         return None
+
+
+DUMP_BYTES = 64 << 20
+
+
+def sample_outputs(arrays):
+    """{name: CUDA tensor} -> {name: float32 host array} for --dump-outputs. The arrays share DUMP_BYTES (less 1 MiB for the
+    .npy headers); one larger than its share becomes a 1-D sample of its flattened elements at positions drawn by a fixed
+    seed and sorted, i.e. the same positions for the same shape on every run."""
+    import torch
+    cap = (DUMP_BYTES - (1 << 20)) // (4 * len(arrays))
+    out = {}
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > cap:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), cap, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        out[name] = t.float().cpu().numpy()
+    return out
+
+
+def write_outputs(path, host_arrays):
+    os.makedirs(path, exist_ok=True)
+    for name, a in host_arrays.items():
+        np.save(os.path.join(path, name + '.npy'), a)
 
 
 def make_video(cfg, n_frames, seed):
@@ -404,11 +435,13 @@ def run_sweep(args, cfg):
     e0.record()
     for _ in range(K):
         flush.zero_()
-        Hm.est_swp_volume_v4(ref, src, c['d'], R, t, cam, c['sigma'])
+        cost = Hm.est_swp_volume_v4(ref, src, c['d'], R, t, cam, c['sigma'])
     e1.record()
     barrier()
     launches = int(L.nrgbd_launch_count())
     ms = max_ms(e0.elapsed_time(e1), world, dev)
+    dumped = sample_outputs({'cost_volume': cost}) if args.dump_outputs and rank == 0 else None
+    del cost
     # kernel-only time of the sweep (events around each call, no flush in between the event pair)
     ks = []
     for _ in range(10):
@@ -449,6 +482,8 @@ def run_sweep(args, cfg):
         }
         if world == 1 and not args.no_cpu_baseline:
             line['cpu_baseline'] = cpu_baseline_subprocess(args)
+        if dumped:
+            write_outputs(args.dump_outputs, dumped)
         _emit(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -561,6 +596,9 @@ def run_engine(args, cfg):
         barrier()
         launches = int(L.nrgbd_launch_count())
         ms_value = max_ms(e0.elapsed_time(e1), world, dev)
+        if args.dump_outputs and rank == 0:
+            last = outs[(Wm + K - 1) % inflight]
+            dumped = sample_outputs({'dmap_cur_refined': last[0], 'bv_cur': last[1], 'depth_lowres': last[2]})
 
         def eager_frame(i):
             flush.zero_()
@@ -649,6 +687,15 @@ def run_engine(args, cfg):
         barrier()
         launches = int(L.nrgbd_launch_count())
         ms_value = max_ms(e0.elapsed_time(e1), world, dev)
+        if args.dump_outputs and rank == 0:
+            i = base + K - 1                            # the last timed step: which chunk, frame and prior slot stream_step used
+            tr, j = trajs[i % inflight], i // inflight
+            if j % n_stream == 0:
+                last = {'dmap_cur_refined': tr['o_ref'], 'depth_lowres': tr['o_dep']}
+            else:
+                last = {'dmap_cur_refined': tr['o_cur'], 'dmap_refined': tr['o_ref'], 'dpv': tr['o_dpv'], 'depth_lowres': tr['o_dep']}
+            last['bv_predict_next'] = tr['priors'][(j + 1) % 2]
+            dumped = sample_outputs(last)
 
         def eager_frame(i):
             stream_step((1 + i % (n_stream - 1)) * inflight, True)      # chunk 0, a steady-state frame
@@ -835,6 +882,8 @@ def run_engine(args, cfg):
                                                   'tflops': round(r_['algorithmic_tflops'], 1)} for r_ in layer_rows[:4]]
         if world == 1 and not args.no_cpu_baseline:
             line['cpu_baseline'] = cpu_baseline_subprocess(args)
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs, dumped)
         _emit(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -857,7 +906,13 @@ def main():
     ap.add_argument('--dev-smem-cap-kb', type=int, default=0, help='development: cap conv_h2 shared memory (co-residency experiment)')
     ap.add_argument('--conv-math', default='f16x3', choices=['fp32', 'tf32x3', 'f16x3'],
                     help='f16x3: tcgen05 kind::f16 on split-fp16 pairs (default); tf32x3: tcgen05 3xTF32; fp32: exact CUDA-core FFMA implicit GEMM')
+    ap.add_argument('--dump-outputs', default=None, metavar='DIR',
+                    help='write what the last timed step returned to DIR/<name>.npy (float32, at most 64 MB in all; larger outputs as a fixed seeded sample)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'engine':
+        ap.error('--dump-outputs applies to the engine arm')
     cfg = CONFIGS[args.config]
     args.warmup = max(args.warmup, 3) if args.impl == 'engine' else args.warmup
     # stdout carries exactly one JSON line: anything a library prints there meanwhile (e.g. NCCL's version banner with

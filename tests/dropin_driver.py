@@ -1,9 +1,10 @@
-"""Runs the reference's OWN inference step (baseline/_ref/code/test_utils/test_KVNet.py:test, unmodified) on the
-engine through neuralrgbd_b200.install_as_reference_modules(), the way test_KVNet.py:159-168,190-250 does:
-construct models.KVNET.KVNET by keyword, wrap in nn.DataParallel, .cuda(), load weights, then stream frames feeding
-each step the prior the previous one returned. Prints one JSON line with the outputs' deviation from the committed
-live-reference fixtures. Executed as a subprocess by tests/test_gpu_dropin.py (keeps the reference's top-level
-module names out of the test process)."""
+"""Runs the inference step of the streaming loop (neuralrgbd_b200.test_utils.test_KVNet.test, the engine's restatement of
+the reference's test_utils/test_KVNet.py:test) on a KVNET built through the reference's import names, the way the
+reference's test_KVNet.py:159-168,190-250 does: install_as_reference_modules() with no checkout registers the engine
+under `models.KVNET`, the model is constructed by keyword, wrapped in nn.DataParallel, .cuda(), loaded with weights,
+then frames are streamed feeding each step the prior the previous one returned. Prints one JSON line with the outputs'
+deviation from the committed live-reference fixtures. Executed as a subprocess by tests/test_gpu_dropin.py (keeps the
+reference's top-level module names out of the test process)."""
 import contextlib
 import io
 import json
@@ -18,17 +19,13 @@ sys.path.insert(0, ROOT)
 
 
 def main():
-    ref_code = sys.argv[1]
-    case_name = sys.argv[2] if len(sys.argv) > 2 else 'kvnet_256_d16'
+    case_name = sys.argv[1] if len(sys.argv) > 1 else 'kvnet_256_d16'
     import neuralrgbd_b200
-    ns = neuralrgbd_b200.install_as_reference_modules(ref_code)
-    import models.KVNET as m_kvnet                     # reference module; KVNET re-pointed to the engine-backed class
-    import test_utils.test_KVNet as ref_step           # the reference's file, unmodified
-    import warping.homography as warp_homo
-    import mutils.misc as m_misc
+    neuralrgbd_b200.install_as_reference_modules()
+    import models.KVNET as m_kvnet                     # the reference's module name, registered to the engine
+    from neuralrgbd_b200.test_utils import test_KVNet as ref_step
     from oracle import planesweep_oracle as O
     from tests import cases
-    assert ref_step.__file__.startswith(os.path.abspath(ref_code)), ref_step.__file__
     c = cases.kvnet_case(case_name)
     cam = cases.cam_for(O.make_cam_intrinsics, c['W'] // 4, c['H'] // 4)
     cam = dict(cam, unit_ray_array_2D=torch.from_numpy(cam['unit_ray_array_2D']),

@@ -1,4 +1,4 @@
-"""Host-side drop-in logic (CPU, no GPU): install_as_reference_modules() against an unmodified reference checkout,
+"""Host-side drop-in logic (CPU, no GPU): install_as_reference_modules() against a reference-shaped checkout,
 and the ownership rules of nn.DataParallel replicas of the engine-backed KVNET (ADVICE r1)."""
 import contextlib
 import io
@@ -8,19 +8,45 @@ import subprocess
 import sys
 
 import numpy as np
-import pytest
 import torch
 
 from tests import cases
 from tests.conftest import ROOT
 
-REF_CODE = os.path.join(ROOT, 'baseline', '_ref', 'code')
+# A stand-in for the `code/` directory of an NVlabs/neuralrgbd checkout: the module names, the symbols the patches
+# touch or must keep, and the cross-imports that matter to the install (warping.homography imports warping.View by
+# `from warping import View`; mutils.misc, models.KVNET, the data loaders and the inference step import the reference
+# modules by their top-level names). Bodies are placeholders: only where each name resolves is checked.
+STUB_CHECKOUT = {
+    'warping/__init__.py': '',
+    'warping/View.py': 'def normalised_pixel_to_ray_array(width=320, height=240, hfov=60, vfov=45, normalize_z=True):\n'
+                       '    raise NotImplementedError\n',
+    'warping/homography.py': 'from warping import View\n' + ''.join(
+        'def %s(*args, **kwargs):\n    raise NotImplementedError\n' % n
+        for n in ('est_swp_volume_v4', 'warp_img_feats_v3', 'warp_img_feats_mgpu', 'resample_vol_cuda', 'get_rel_extrinsicM',
+                  'back_warp_th_Rt', 'back_warp_th_Rt_msrc')),
+    'mutils/__init__.py': '',
+    'mutils/misc.py': 'import warping.View as View\nimport warping.homography as warp_homo\n' + ''.join(
+        'def %s(*args, **kwargs):\n    raise NotImplementedError\n' % n
+        for n in ('depth_val_regression', 'valid_dpv', 'get_entries_list_dict', 'm_makedir', 'save_ScenePathInfo',
+                  'split_frame_list')),
+    'models/__init__.py': '',
+    'models/KVNET.py': 'import warping.homography as warp_homo\nimport mutils.misc as m_misc\n\n\nclass KVNET:\n    pass\n',
+    'mdataloader/__init__.py': '',
+    'mdataloader/scanNet.py': 'import warping.View as View\n',
+    'test_utils/__init__.py': '',
+    'test_utils/test_KVNet.py': 'import warping.homography as warp_homo\nimport mutils.misc as m_misc\n\n\n'
+                                'def test(*args, **kwargs):\n    return warp_homo.resample_vol_cuda(*args, **kwargs)\n',
+}
 
 
-def _have_ref():
-    if not os.path.isdir(REF_CODE) and os.path.isdir('/root/reference/code'):
-        subprocess.run([sys.executable, os.path.join(ROOT, 'baseline', 'fetch_reference.py')], check=True, capture_output=True)
-    return os.path.isdir(REF_CODE)
+def _stub_checkout(root):
+    code = os.path.join(str(root), 'code')
+    for rel, text in STUB_CHECKOUT.items():
+        os.makedirs(os.path.dirname(os.path.join(code, rel)), exist_ok=True)
+        with open(os.path.join(code, rel), 'w') as f:
+            f.write(text)
+    return code
 
 
 INSTALL_PROBE = r'''
@@ -48,11 +74,10 @@ print(json.dumps(out))
 '''
 
 
-def test_install_patches_the_reference_modules_in_place():
-    if not _have_ref():
-        pytest.skip('baseline/_ref not present (run baseline/fetch_reference.py in the build container)')
+def test_install_patches_the_reference_modules_in_place(tmp_path):
+    REF_CODE = _stub_checkout(tmp_path)
     r = subprocess.run([sys.executable, '-c', INSTALL_PROBE % dict(root=ROOT, ref=REF_CODE)], capture_output=True, text=True,
-                       timeout=600)
+                       timeout=600, cwd=str(tmp_path))
     assert r.returncode == 0, r.stderr[-2000:]
     out = json.loads(r.stdout.strip().splitlines()[-1])
     assert out['homography_file'].startswith(REF_CODE) and out['misc_file'].startswith(REF_CODE)      # reference modules stay

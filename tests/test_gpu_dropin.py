@@ -1,6 +1,6 @@
 """Drop-in boundary on the GPU (SURVEY 8b; VERDICT r1 weak #4, ADVICE r1 high):
- * the reference's own `test_utils/test_KVNet.py:test` (baseline/_ref, unmodified) runs on the engine after
-   install_as_reference_modules() and reproduces the live-reference fixtures;
+ * the inference step `test_utils.test_KVNet.test` streams frames on a KVNET built through the reference's
+   `models.KVNET` name (install_as_reference_modules()) and nn.DataParallel, and reproduces the live-reference fixtures;
  * a real nn.DataParallel replica (torch.nn.parallel.replicate) of the engine-backed KVNET runs a forward, and
    freeing it leaves the owner's engines usable.
 """
@@ -20,13 +20,10 @@ from tests import cases
 from tests.conftest import ROOT, maxabs
 
 pytestmark = pytest.mark.gpu
-REF_CODE = os.path.join(ROOT, 'baseline', '_ref', 'code')
 
 
-def test_reference_inference_step_runs_unmodified_on_the_engine():
-    if not os.path.isdir(REF_CODE):
-        pytest.skip('baseline/_ref not shipped')
-    r = subprocess.run([sys.executable, os.path.join(ROOT, 'tests', 'dropin_driver.py'), REF_CODE, 'kvnet_256_d16'],
+def test_reference_inference_step_runs_on_the_engine():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, 'tests', 'dropin_driver.py'), 'kvnet_256_d16'],
                        capture_output=True, text=True, timeout=900)
     assert r.returncode == 0, (r.stdout[-1500:], r.stderr[-3000:])
     out = json.loads(r.stdout.strip().splitlines()[-1])
